@@ -6,6 +6,7 @@ backbone (Resnet18_8s) + RANSAC vote (ransac_voting_layer_v3).
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (rank 0)
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --config 4 | --config 5                  # another BASELINE config as the headline
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs to DIR/*.npy
 
 One "step" = one batch of 16 synthetic 480x640 images per GPU (BASELINE config 2, the headline at
 every N so that the per-GPU work is fixed -- "weak" scaling):
@@ -358,11 +359,13 @@ def run_reference_arm(args):
     step, cores = _cpu_path()
     for _ in range(max(1, min(args.warmup, 2))):
         step()
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     t0 = time.perf_counter()
     for _ in range(steps):
-        step()
+        kp = step()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"keypoints": kp})
     val = steps / dt
     line = {
         "impl": "reference", "metric": "images/sec (480x640, K=9) backbone+vote", "value": round(val, 4),
@@ -379,10 +382,28 @@ def run_reference_arm(args):
 
 
 # ----------------------------------------------------------------------------- main
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dst, arrays):
+    """Writes each array as dst/<name>.npy in float32 (float64 stays float64), so that two builds run with
+    the same arguments -- hence the same inputs -- can be compared output for output."""
+    os.makedirs(dst, exist_ok=True)
+    out = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        out[name] = a if a.dtype == np.float64 else a.astype(np.float32)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES} byte limit")
+    for name, a in out.items():
+        np.save(os.path.join(dst, name + ".npy"), a)
+
+
 def measure(torch, dist, pd, pipe, xs, hosts, batch, k, steps, warmup, world, sampler=None, rank=0):
     """One configuration, two ways: K steps on device-resident inputs, and the same K steps through
     PoseKeypointPipeline.run from pinned host buffers.  Returns per-rank (ms_device, ms_e2e, launches,
-    clocks or None)."""
+    clocks or None, outputs): outputs = what the last step of each timed loop returned, by name."""
     from pvnet_b200 import _native
     with_cov = pipe.with_cov
 
@@ -417,11 +438,12 @@ def measure(torch, dist, pd, pipe, xs, hosts, batch, k, steps, warmup, world, sa
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(steps):
-            full_step(xs[i % 3])
+            r = full_step(xs[i % 3])
         e1.record()
         barrier()
         launches = _native.launch_count()
         ms_dev = e0.elapsed_time(e1)
+        outputs = {"keypoints": r[0].cpu(), "covariance": r[1].cpu()} if with_cov else {"keypoints": r.cpu()}
 
         kp_hosts = [torch.empty([batch, k, 2]).pin_memory() for _ in range(steps)]
         cov_hosts = [torch.empty([batch, k, 2, 2]).pin_memory() for _ in range(steps)] if with_cov else None
@@ -438,7 +460,10 @@ def measure(torch, dist, pd, pipe, xs, hosts, batch, k, steps, warmup, world, sa
         barrier()
         ms_e2e = f0.elapsed_time(f1)
         clocks = sampler.stop() if (sampler is not None and rank == 0) else None
-    return ms_dev, ms_e2e, launches, clocks
+    outputs["e2e_keypoints"] = kp_hosts[-1]
+    if with_cov:
+        outputs["e2e_covariance"] = cov_hosts[-1]
+    return ms_dev, ms_e2e, launches, clocks, outputs
 
 
 def main():
@@ -453,7 +478,13 @@ def main():
     ap.add_argument("--with-cov", action="store_true", help="same as --config 4")
     ap.add_argument("--e2e-input", default="u8", choices=["u8", "f32"],
                     help="host buffers of the e2e arm: raw uint8 HWC images normalised on the device, or float32 NCHW")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step returned as DIR/<name>.npy (rank 0): "
+                         "keypoints (and covariance) of the device-resident arm, e2e_* of the end-to-end arm, "
+                         "config4_* for config 4's measurement in the same line")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.with_cov:
         args.config = 4
@@ -494,12 +525,15 @@ def main():
     fg = calibrate_foreground(torch, net, xs[0], cfg["fg"])
 
     pipe = make_pipe(net, cfg)
-    ms_total, ms_e2e, launches, clocks = measure(torch, dist, pd, pipe, xs, hosts, batch, k, args.steps, args.warmup, world,
-                                                 ClockSampler(local), rank)
+    ms_total, ms_e2e, launches, clocks, outputs = measure(torch, dist, pd, pipe, xs, hosts, batch, k, args.steps,
+                                                          args.warmup, world, ClockSampler(local), rank)
     extra = None
     if args.config == 2:                             # config 4's per-GPU workload in the same process, same N
         pipe4 = make_pipe(net, CONFIGS[4])
         extra = measure(torch, dist, pd, pipe4, xs, hosts, batch, k, args.steps, args.warmup, world)
+        outputs.update({"config4_" + name: a for name, a in extra[4].items()})
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
 
     vals = [ms_total, ms_e2e] + ([extra[0], extra[1]] if extra else [0.0, 0.0])
     t = torch.tensor(vals, device=dev, dtype=torch.float64)

@@ -1,20 +1,32 @@
-"""GPU box only: the reference's OWN CUDA kernels (oracle/_ref, compiled verbatim from
-/root/reference by oracle/Makefile in the authoring container) against the oracle and
-against the product.  This is what pins the oracle (SURVEY.md §8c) and what measures
-"within 1e-4 of the reference CUDA layer"."""
+"""The reference's OWN CUDA kernels against the oracle and against the product.  What those kernels
+(oracle/_ref: the reference's ransac_voting_kernel.cu compiled verbatim by oracle/Makefile, driven by
+oracle/ref_cuda.py with the reference's torch ops) computed on the inputs below is stored in
+tests/golden/ref_cuda_kernels.npz and ref_cuda_layer.npz by tests/golden/make_golden_ref_cuda.py
+(large exact-match arrays as digests: tests.helpers.digest).
+This is what pins the oracle (SURVEY.md §8c, CPU) and what measures "within 1e-4 of the reference
+CUDA layer" (GPU)."""
+import os
+
 import numpy as np
 import pytest
 import torch
 
 from oracle import pvnet_oracle as po
-from oracle import ref_cuda
 from pvnet_b200 import ransac_voting_gpu as rv
 from pvnet_b200 import synthetic as syn
-from tests.helpers import cfg1_inputs, demo_fixture
+from tests.helpers import EDGE_THRESHOLDS, REF_LAYER_CASES, cfg1_inputs, digest, edge_kernel_inputs, ref_layer_inputs
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not ref_cuda.available(), reason="oracle/_ref/libpvnet_refcuda.so not built")]
 DEV = "cuda:0"
+
+
+@pytest.fixture(scope="module")
+def kernels(golden_dir):
+    return np.load(os.path.join(golden_dir, "ref_cuda_kernels.npz"))
+
+
+@pytest.fixture(scope="module")
+def layer(golden_dir):
+    return np.load(os.path.join(golden_dir, "ref_cuda_layer.npz"))
 
 
 def _dev_inputs(mask_np, field_np):
@@ -25,65 +37,46 @@ def _dev_inputs(mask_np, field_np):
 
 
 @pytest.mark.parametrize("kind", ["random", "planted"])
-def test_reference_kernels_pin_the_oracle(kind):
+def test_reference_kernels_pin_the_oracle(kernels, kind):
     mask, field, idxs = cfg1_inputs(kind)
     coords, direct = po.compact(mask.astype(np.uint8), syn.as_reference_view(field[None])[0])
-    d, c, i = (torch.from_numpy(a).to(DEV) for a in (direct, coords, idxs))
-    hyp = ref_cuda.generate_hypothesis(d, c, i)
+    hyp = kernels[f"cfg1_{kind}_hyp"]
     ohyp = po.generate_hypothesis_kernel(direct, coords, idxs)
-    assert np.array_equal(hyp.cpu().numpy().view(np.uint32), ohyp.view(np.uint32))
-    inl = torch.zeros([128, 9, 10000], dtype=torch.uint8, device=DEV)
-    ref_cuda.voting_for_hypothesis(d, c, hyp, inl, 0.99)
-    assert np.array_equal(inl.sum(2).cpu().numpy().astype(np.int32), po.vote_counts(direct, coords, ohyp, 0.99))
-    assert np.array_equal(inl[:8].cpu().numpy(), po.voting_for_hypothesis_kernel(direct, coords, ohyp[:8], 0.99))
+    assert np.array_equal(hyp.view(np.uint32), ohyp.view(np.uint32))
+    assert np.array_equal(kernels[f"cfg1_{kind}_counts"], po.vote_counts(direct, coords, ohyp, 0.99))
+    assert kernels[f"cfg1_{kind}_inliers8"] == digest(po.voting_for_hypothesis_kernel(direct, coords, ohyp[:8], 0.99))
 
 
-def test_reference_kernels_pin_the_oracle_on_edge_values():
-    rng = np.random.default_rng(0)
-    tn, vn, hn = 4096, 3, 64
-    direct = rng.standard_normal((tn, vn, 2)).astype(np.float32)
-    direct[:200] *= 1e-6            # around the 1e-6 norm test
-    direct[200:300] = 0
-    direct[300:400, :, 1] = direct[300:400, :, 0]          # near-parallel families
-    coords = np.stack([rng.integers(0, 640, tn), rng.integers(0, 480, tn)], 1).astype(np.float32)
-    idxs = rng.integers(0, tn, (hn, vn, 2), dtype=np.int32)
-    d, c, i = (torch.from_numpy(a).to(DEV) for a in (direct, coords, idxs))
-    hyp = ref_cuda.generate_hypothesis(d, c, i)
+def test_reference_kernels_pin_the_oracle_on_edge_values(kernels):
+    direct, coords, idxs, extra = edge_kernel_inputs()
     ohyp = po.generate_hypothesis_kernel(direct, coords, idxs)
-    assert np.array_equal(hyp.cpu().numpy().view(np.uint32), ohyp.view(np.uint32))
+    assert np.array_equal(kernels["edge_hyp"].view(np.uint32), ohyp.view(np.uint32))
     # also hypotheses ON pixels (norm2 == 0) and far away
-    extra = np.concatenate([coords[:32, None, :].repeat(vn, 1), np.full((8, vn, 2), 3e7, np.float32)]).astype(np.float32)
-    for thresh in (0.99, 0.5, -0.25):
-        for hp in (ohyp, extra):
-            inl = torch.zeros([hp.shape[0], vn, tn], dtype=torch.uint8, device=DEV)
-            ref_cuda.voting_for_hypothesis(d, c, torch.from_numpy(hp).to(DEV), inl, thresh)
-            assert np.array_equal(inl.cpu().numpy(), po.voting_for_hypothesis_kernel(direct, coords, hp, thresh))
+    for t, thresh in enumerate(EDGE_THRESHOLDS):
+        for j, hp in enumerate((ohyp, extra)):
+            assert kernels[f"edge_inliers_{t}_{j}"] == digest(po.voting_for_hypothesis_kernel(direct, coords, hp, thresh))
 
 
-def _product_vs_reference_layer(mask_np, field_np, hn, thresh, max_num=30000, label=""):
-    """Runs the reference layer (its own kernels + its torch ops, fp32 refit), the same
-    with the refit ops in fp64, and the product, all from torch.manual_seed(0).
-    Asserts fixed-seed parity of samples / hypotheses / counts, and that the product is
-    within 1e-4 of the reference layer once the reference's fp32 refit rounding is taken
-    out (fp64 run).  Returns the gaps."""
-    mask, vertex = _dev_inputs(mask_np, field_np)
-    rec = []
+def _product_vs_reference_layer(layer, name, label=""):
+    """Runs the product from torch.manual_seed(0) and compares it with the reference layer (its own
+    kernels + its torch ops) run from the same seed, with its stock fp32 refit and with the refit ops
+    in fp64.  Asserts fixed-seed parity of samples / hypotheses / counts, and that the product is
+    within 1e-4 of the reference layer once the reference's fp32 refit rounding is taken out (fp64
+    run).  Returns the gaps."""
+    mask, vertex = _dev_inputs(*ref_layer_inputs(name))
     torch.manual_seed(0)
-    ref_kp = ref_cuda.layer_v3(mask, vertex, hn, inlier_thresh=thresh, max_num=max_num, record=rec)
-    torch.manual_seed(0)
-    ref_kp64 = ref_cuda.layer_v3(mask, vertex, hn, inlier_thresh=thresh, max_num=max_num,
-                                 refit_dtype=torch.float64)
-    torch.manual_seed(0)
-    kp, dbg = rv.ransac_voting_layer_v3(mask, vertex, hn, inlier_thresh=thresh, max_num=max_num, return_debug=True)
-    for bi, r in enumerate(rec):
-        if r is None:
+    kp, dbg = rv.ransac_voting_layer_v3(mask, vertex, REF_LAYER_CASES[name]["hn"], inlier_thresh=0.99,
+                                        max_num=30000, return_debug=True)
+    for bi, tn in enumerate(layer[f"{name}_tn"]):
+        if tn < 0:
             continue
         # fixed-seed parity: same samples drawn, same counts, same winner
-        assert torch.equal(dbg["idxs"][bi], r["idxs"]), "RNG stream differs from the reference's"
-        assert int(dbg["tn"][bi]) == r["tn"]
-        assert torch.equal(dbg["counts"][bi].long(), r["counts"]), "inlier counts differ from the reference layer"
-        assert torch.equal(dbg["hyp"][bi], r["hyp"])
-    kp, ref_kp, ref_kp64 = kp.cpu().numpy(), ref_kp.cpu().numpy(), ref_kp64.cpu().numpy()
+        assert digest(dbg["idxs"][bi].cpu().numpy()) == layer[f"{name}_idxs"][bi], "RNG stream differs from the reference's"
+        assert int(dbg["tn"][bi]) == tn
+        assert digest(dbg["counts"][bi].cpu().numpy()) == layer[f"{name}_counts"][bi], \
+            "inlier counts differ from the reference layer"
+        assert digest(dbg["hyp"][bi].cpu().numpy()) == layer[f"{name}_hyp"][bi]
+    kp, ref_kp, ref_kp64 = kp.cpu().numpy(), layer[f"{name}_kp"], layer[f"{name}_kp64"]
     gap32 = np.abs(kp - ref_kp).max()
     gap64 = np.abs(kp - ref_kp64).max()
     noise = np.abs(ref_kp - ref_kp64).max()
@@ -95,94 +88,69 @@ def _product_vs_reference_layer(mask_np, field_np, hn, thresh, max_num=30000, la
     return gap32, gap64, noise
 
 
-def test_fixed_seed_parity_with_reference_layer_config1():
-    mask, field, _ = cfg1_inputs("planted")
-    _product_vs_reference_layer(np.stack([mask, mask]), np.stack([field, field]), 128, 0.99,
+def _cov_vs_reference_layer(layer, name):
+    """The product's estimate_voting_distribution_with_mean against the reference's, from the same torch
+    seed and the same mean: samples, counts, covariances.  Returns (ours, the reference's)."""
+    mask, vertex = _dev_inputs(*ref_layer_inputs(name))
+    seed, hn, min_hyp = REF_LAYER_CASES[name]["cov"]
+    mean = torch.from_numpy(layer[f"{name}_mean"]).to(DEV)
+    torch.manual_seed(seed)
+    _, cov, dbg = rv.estimate_voting_distribution_with_mean(mask, vertex, mean, round_hyp_num=hn, min_hyp_num=min_hyp,
+                                                            inlier_thresh=0.99, max_num=30000, return_debug=True)
+    for bi in range(mask.shape[0]):
+        assert digest(dbg["idxs"][bi].cpu().numpy()) == layer[f"{name}_cov_idxs"][bi], \
+            "RNG stream differs from the reference's"
+        assert digest(dbg["counts"][bi].cpu().numpy()) == layer[f"{name}_cov_counts"][bi], \
+            "inlier counts differ from the reference layer"
+    ref_cov = torch.from_numpy(layer[f"{name}_cov"]).to(DEV)
+    assert torch.allclose(cov, ref_cov, atol=1e-4, rtol=1e-4), (cov - ref_cov).abs().max().item()
+    return cov, ref_cov
+
+
+@pytest.mark.gpu
+def test_fixed_seed_parity_with_reference_layer_config1(layer):
+    _product_vs_reference_layer(layer, "config1",
                                 label="config1 planted, tn=10000, K=9 (odd keypoints 260 px outside the mask)")
 
 
-def test_fixed_seed_parity_with_reference_layer_demo():
+@pytest.mark.gpu
+def test_fixed_seed_parity_with_reference_layer_demo(layer):
     """The reference's own demo fixture (well conditioned: keypoints inside the object)."""
-    mask, field, pts = demo_fixture()
-    gap32, _, _ = _product_vs_reference_layer(mask[None], field[None], 512, 0.99, label="demo fixture, tn=2289")
+    gap32, _, _ = _product_vs_reference_layer(layer, "demo", label="demo fixture, tn=2289")
     assert gap32 <= 1e-3
 
 
-def test_fixed_seed_parity_near_keypoints():
+@pytest.mark.gpu
+def test_fixed_seed_parity_near_keypoints(layer):
     """Keypoints inside the mask (R=20 px): the best-conditioned case."""
-    mask = syn.disc_mask(3000)
-    rng = np.random.default_rng(5)
-    kps = np.stack([320 + 20 * np.cos(np.arange(9)), 240 + 20 * np.sin(np.arange(9))], 1)
-    ys, xs = np.mgrid[0:480, 0:640].astype(np.float64)
-    field = np.zeros((18, 480, 640), np.float32)
-    for j in range(9):
-        dx, dy = kps[j, 0] - xs, kps[j, 1] - ys
-        n = np.sqrt(dx * dx + dy * dy) + 1e-3
-        eps = rng.normal(0, 0.03, size=dx.shape)
-        field[2 * j] = (np.cos(eps) * dx / n - np.sin(eps) * dy / n) * (mask != 0)
-        field[2 * j + 1] = (np.sin(eps) * dx / n + np.cos(eps) * dy / n) * (mask != 0)
-    gap32, _, _ = _product_vs_reference_layer(mask[None], field[None], 256, 0.99, label="near keypoints, tn=3000")
+    gap32, _, _ = _product_vs_reference_layer(layer, "near", label="near keypoints, tn=3000")
     assert gap32 <= 1e-3
 
 
-def test_fixed_seed_parity_with_subsampling():
-    masks = np.stack([syn.disc_mask(40000), syn.disc_mask(3), syn.disc_mask(9000)])
-    fields = np.stack([syn.planted_field(masks[i], 9, 40 + i)[0] for i in range(3)])
-    _product_vs_reference_layer(masks, fields, 256, 0.99, max_num=30000, label="subsampled 40000->~30000")
+@pytest.mark.gpu
+def test_fixed_seed_parity_with_subsampling(layer):
+    _product_vs_reference_layer(layer, "subsampled", label="subsampled 40000->~30000")
 
 
-def test_covariance_fixed_seed_parity():
-    masks = np.stack([syn.disc_mask(7000), syn.disc_mask(12000)])
-    fields = np.stack([syn.planted_field(masks[i], 9, 60 + i, sigma=0.05)[0] for i in range(2)])
-    mask, vertex = _dev_inputs(masks, fields)
-    torch.manual_seed(1)
-    mean = rv.ransac_voting_layer_v3(mask, vertex, 256, inlier_thresh=0.99)
-    rec = []
-    torch.manual_seed(2)
-    _, ref_cov = ref_cuda.layer_cov_with_mean(mask, vertex, mean, round_hyp_num=128, min_hyp_num=512,
-                                              inlier_thresh=0.99, record=rec)
-    torch.manual_seed(2)
-    _, cov, dbg = rv.estimate_voting_distribution_with_mean(mask, vertex, mean, round_hyp_num=128, min_hyp_num=512,
-                                                            inlier_thresh=0.99, return_debug=True)
-    for bi, r in enumerate(rec):
-        assert torch.equal(dbg["idxs"][bi], r["idxs"])
-        assert torch.equal(dbg["counts"][bi].long(), r["counts"])
+@pytest.mark.gpu
+def test_covariance_fixed_seed_parity(layer):
+    cov, ref_cov = _cov_vs_reference_layer(layer, "covariance")
     gap = (cov - ref_cov).abs()
     print(f"\n[reference-layer gap] covariance: max abs {gap.max().item():.3e}, "
           f"max rel {(gap / ref_cov.abs().clamp_min(1e-6)).max().item():.3e}, |cov| max {ref_cov.abs().max().item():.3e}")
-    assert torch.allclose(cov, ref_cov, atol=1e-4, rtol=1e-4)
 
 
-def _cov_vs_reference_layer(masks, fields, hn, min_hyp, thresh, max_num, seed):
-    mask, vertex = _dev_inputs(masks, fields)
-    torch.manual_seed(seed)
-    mean = rv.ransac_voting_layer_v3(mask, vertex, hn, inlier_thresh=thresh, max_num=max_num)
-    rec = []
-    torch.manual_seed(seed + 1)
-    _, ref_cov = ref_cuda.layer_cov_with_mean(mask, vertex, mean, round_hyp_num=hn, min_hyp_num=min_hyp,
-                                              inlier_thresh=thresh, max_num=max_num, record=rec)
-    torch.manual_seed(seed + 1)
-    _, cov, dbg = rv.estimate_voting_distribution_with_mean(mask, vertex, mean, round_hyp_num=hn, min_hyp_num=min_hyp,
-                                                            inlier_thresh=thresh, max_num=max_num, return_debug=True)
-    for bi, r in enumerate(rec):
-        assert torch.equal(dbg["idxs"][bi], r["idxs"]), "RNG stream differs from the reference's"
-        assert torch.equal(dbg["counts"][bi].long(), r["counts"]), "inlier counts differ from the reference layer"
-    assert torch.allclose(cov, ref_cov, atol=1e-4, rtol=1e-4), (cov - ref_cov).abs().max().item()
-
-
-def test_config4_shape_fixed_seed_vs_reference_layer():
+@pytest.mark.gpu
+def test_config4_shape_fixed_seed_vs_reference_layer(layer):
     """BASELINE config 4 per image (K=9, 20000 px, v3(256) + with_mean(256, 4096), thresh 0.99) against the reference's
     own kernels + torch ops under the same torch seed: samples, counts, keypoints, covariances."""
-    masks = np.stack([syn.disc_mask(20000)])
-    fields = np.stack([syn.planted_field(masks[0], 9, 4400, sigma=0.05)[0]])
-    _product_vs_reference_layer(masks, fields, 256, 0.99, label="config 4 shape, tn=20000, K=9, 256 hyp")
-    _cov_vs_reference_layer(masks, fields, 256, 4096, 0.99, 30000, seed=44)
+    _product_vs_reference_layer(layer, "config4", label="config 4 shape, tn=20000, K=9, 256 hyp")
+    _cov_vs_reference_layer(layer, "config4")
 
 
-def test_config5_shape_fixed_seed_vs_reference_layer():
+@pytest.mark.gpu
+def test_config5_shape_fixed_seed_vs_reference_layer(layer):
     """BASELINE config 5 per image (K=17, 92160 px subsampled to ~30000 by the reference's own uniform_ draw,
     v3(1024) + with_mean(1024, 1024))."""
-    masks = np.stack([syn.disc_mask(92160)])
-    fields = np.stack([syn.planted_field(masks[0], 17, 5500, sigma=0.05)[0]])
-    _product_vs_reference_layer(masks, fields, 1024, 0.99, max_num=30000, label="config 5 shape, 92160 px -> ~30000, K=17, 1024 hyp")
-    _cov_vs_reference_layer(masks, fields, 1024, 1024, 0.99, 30000, seed=55)
+    _product_vs_reference_layer(layer, "config5", label="config 5 shape, 92160 px -> ~30000, K=17, 1024 hyp")
+    _cov_vs_reference_layer(layer, "config5")

@@ -13,7 +13,7 @@ from lib.ransac_voting_gpu_layer.ransac_voting_gpu import (estimate_voting_distr
                                                            ransac_voting_layer_v4)
 from oracle import pvnet_oracle as po
 from pvnet_b200 import synthetic as syn
-from tests.helpers import variant_inputs
+from tests.helpers import digest, variant_inputs, vp_inputs
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -126,21 +126,9 @@ def test_v4_full_size():
 
 
 # ---------------------------------------------------------------- vanishing-point pair (ransac_voting_kernel.cu:170-351)
-def _vp_inputs(seed, tn=3000, vn=4, hn=96):
-    rng = np.random.default_rng(seed)
-    direct = rng.standard_normal((tn, vn, 2)).astype(np.float32)
-    direct[:100] *= 1e-6                                # around the 1e-6 norm test
-    direct[100:150] = 0
-    direct[150:300, :, 1] = direct[150:300, :, 0]       # parallel families: z ~ 0 (points at infinity)
-    coords = np.stack([rng.integers(0, 640, tn), rng.integers(0, 480, tn)], 1).astype(np.float32)
-    idxs = rng.integers(0, tn, (hn, vn, 2), dtype=np.int32)
-    return direct, coords, idxs
-
-
-def test_vanishing_point_pair_bit_exact_vs_oracle_and_reference_kernels():
-    from oracle import ref_cuda
+def test_vanishing_point_pair_bit_exact_vs_oracle_and_reference_kernels(golden_dir):
     from pvnet_b200 import ransac_voting as ext
-    direct, coords, idxs = _vp_inputs(21)
+    direct, coords, idxs = vp_inputs(21)
     d, c, i = (torch.from_numpy(a).to(DEV) for a in (direct, coords, idxs))
     hyp = ext.generate_hypothesis_vanishing_point(d, c, i)
     ohyp = po.generate_hypothesis_vanishing_point_kernel(direct, coords, idxs)
@@ -153,14 +141,12 @@ def test_vanishing_point_pair_bit_exact_vs_oracle_and_reference_kernels():
         assert np.array_equal(inl.cpu().numpy(), oinl)
         assert np.array_equal(cnt.cpu().numpy(), oinl.sum(2))
         assert oinl.sum() > 1000
-    if ref_cuda.available() and hasattr(ref_cuda.lib(), "pvref_generate_hypothesis_vp"):
-        rhyp = ref_cuda.generate_hypothesis_vanishing_point(d, c, i)     # the reference's own kernels pin both
-        assert torch.equal(rhyp.view(torch.int32), hyp.view(torch.int32))
-        rinl = torch.zeros([96, 4, 3000], dtype=torch.uint8, device=DEV)
-        ref_cuda.voting_for_hypothesis_vanishing_point(d, c, rhyp, rinl, 0.99)
-        inl = torch.zeros([96, 4, 3000], dtype=torch.uint8, device=DEV)
-        ext.voting_for_hypothesis_vanishing_point(d, c, hyp, inl, 0.99)
-        assert torch.equal(rinl, inl)
+    # the reference's own kernels pin both (tests/golden/make_golden_ref_cuda.py)
+    ref = np.load(os.path.join(golden_dir, "ref_cuda_kernels.npz"))
+    assert np.array_equal(ref["vp_hyp"].view(np.int32), hyp.cpu().numpy().view(np.int32))
+    inl = torch.zeros([96, 4, 3000], dtype=torch.uint8, device=DEV)
+    ext.voting_for_hypothesis_vanishing_point(d, c, hyp, inl, 0.99)
+    assert ref["vp_inliers"] == digest(inl.cpu().numpy())
 
 
 def test_v2_against_reference_fixture(gold):
