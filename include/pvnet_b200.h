@@ -25,6 +25,8 @@
  *   tools/train_linemod.py:119-130                                UncertaintyEvalWrapper.forward (v3 + with_mean)
  *   lib/utils/extend_utils/extend_utils.py:63-114                 uncertainty_pnp (+ evaluation_utils.py:165-201)
  *   lib/networks/model_repository.py:64-80                        Resnet18_8s.forward
+ *   lib/utils/extend_utils/src/nearest_neighborhood.cu:48-163     findNearestPointIdxLauncher
+ *   lib/utils/evaluation_utils.py:54-141                          Evaluator's metric methods
  * INTEGRATION.md shows the ctypes binding the reference's Python wrapper uses.
  */
 #ifndef PVNET_B200_H_
@@ -253,6 +255,56 @@ PVNET_API int pvnet_generate_hypothesis_vanishing_point(const float *direct, con
 PVNET_API int pvnet_voting_for_hypothesis_vanishing_point(const float *direct, const float *coords, const float *hypo,
                                                           uint8_t *inliers, int32_t *counts, int tn, int vn, int hn,
                                                           float inlier_thresh, pvnet_stream_t stream);
+
+/* ------------------------------------------------------------------ pose-accuracy metrics
+ *
+ * pvnet_find_nearest_point_idx: batched form of extend_utils.py:39-60 `find_nearest_point_idx(ref_pts,
+ *   que_pts)`, the index the reference kernel findNearestPoint{2D,3D}IdxKernel (nearest_neighborhood.cu:48-117)
+ *   returns, bit for bit:
+ *     ref   f32 [b,pn1,dim]  the points searched
+ *     que   f32 [b,pn2,dim]  one answer per query point
+ *     idxs  int32 [b,pn2]    out: for que[bi,j], the i minimising |ref[bi,i] - que[bi,j]|^2
+ *     dim   2 or 3;  exclude_self != 0 skips i == j (the launcher's last argument, :123-163)
+ *   The distance is the reference's rounding sequence (d = ref - que; 2-D fma(dx,dx,dy*dy), 3-D
+ *   fma(dz,dz,fma(dx,dx,dy*dy)), DESIGN.md §2); the selection starts at (FLT_MAX, 0) and replaces only on a
+ *   strict `<` in increasing index: the lowest index wins a tie, NaN and +inf are never chosen, a query with
+ *   no finite distance gets 0.  Offsets are 64-bit.  b <= 65535.  No workspace. */
+PVNET_API int pvnet_find_nearest_point_idx(const float *ref, const float *que, int32_t *idxs, int b, int pn1, int pn2,
+                                           int dim, int exclude_self, pvnet_stream_t stream);
+
+/* Flags of pvnet_pose_metrics. */
+enum {
+    PVNET_METRICS_SYM_ADD = 1,  /* ADD-S: add_metric_sym (evaluation_utils.py:119-130) instead of add_metric */
+    PVNET_METRICS_SYM_PROJ = 2, /* projection_2d_sym (:83-89) instead of projection_2d (:75-81) */
+    PVNET_METRICS_PRED_F32 = 4, /* pose_pred holds float32 values: its cloud is float32, as numpy makes it */
+    PVNET_METRICS_GT_F32 = 8    /* pose_gt holds float32 values (the data loader's dtype): likewise */
+};
+
+/* pvnet_pose_metrics: the metric methods of the reference's Evaluator (evaluation_utils.py:64-141) for a batch
+ * of b images of one object, fp64, deterministic (fixed-order sums):
+ *   pose_pred, pose_gt  f64 [b,3,4] (R | t)
+ *   model_points        f32 [pn,3] (the object model, metres)
+ *   camera_matrix       HOST array of 9 doubles, one K for all images; OR
+ *   camera_matrices     f64 [b,3,3] on the device, one K per image (`use_camera_intrinsic`); pass NULL for the other
+ *   flags               PVNET_METRICS_* above
+ *   values              out f64 [b,4]:
+ *     [0] add_dist        mean_X |(R_p X + t_p) - (R_g X + t_g)|                        add_metric      :91-117
+ *                         with SYM_ADD: mean over target points of the distance to the nearest predicted point,
+ *                         the index searched on both clouds rounded to f32 (find_nearest_point_distance :54-62)
+ *     [1] proj_mean_diff  mean 2-D distance of the two projections (Projector.project_K)  projection_2d   :75-81
+ *                         with SYM_PROJ: the same nearest-point rule in 2-D              projection_2d_sym :83-89
+ *     [2] trans_cm        |t_p - t_g| * 100                                              cm_degree_5_metric :132-141
+ *     [3] rot_deg         degrees(arccos((min(tr(R_p R_g^T), 3) - 1) / 2)); no lower clamp (NaN below -1)
+ *   ok                  out u8 [b,3]: add_dist < add_threshold (the reference's percentage * diameter),
+ *                       proj_mean_diff < proj_threshold (5), trans_cm < cm_threshold && rot_deg < deg_threshold (5, 5)
+ *   workspace           pvnet_pose_metrics_workspace_bytes(b, pn, flags) bytes (0 without a SYM flag: may be NULL)
+ * One launch, plus one cloud launch and one pvnet_find_nearest_point_idx launch per SYM flag. */
+PVNET_API int pvnet_pose_metrics_workspace_bytes(int b, int pn, int flags, size_t *bytes);
+PVNET_API int pvnet_pose_metrics(const double *pose_pred, const double *pose_gt, const float *model_points,
+                                 const double camera_matrix[9], const double *camera_matrices, int b, int pn, int flags,
+                                 double add_threshold, double proj_threshold, double cm_threshold,
+                                 double deg_threshold, double *values, uint8_t *ok, void *workspace,
+                                 size_t workspace_bytes, pvnet_stream_t stream);
 
 /* Number of kernels this library has launched on the calling thread since the last
  * reset (bench.py's "gpu_launches"). */

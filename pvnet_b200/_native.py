@@ -53,6 +53,11 @@ SIGNATURES = {
     "pvnet_covariance_to_weights": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),
     "pvnet_uncertainty_pnp": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, ctypes.POINTER(ctypes.c_double), c_int, c_int,
                                       c_void_p, c_void_p, c_void_p]),
+    "pvnet_find_nearest_point_idx": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "pvnet_pose_metrics_workspace_bytes": (c_int, [c_int, c_int, c_int, ctypes.POINTER(c_size_t)]),
+    "pvnet_pose_metrics": (c_int, [c_void_p, c_void_p, c_void_p, ctypes.POINTER(ctypes.c_double), c_void_p, c_int, c_int,
+                                   c_int, ctypes.c_double, ctypes.c_double, ctypes.c_double, ctypes.c_double, c_void_p,
+                                   c_void_p, c_void_p, c_size_t, c_void_p]),
     "pvnet_generate_hypothesis": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "pvnet_voting_for_hypothesis": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_float,
                                             c_void_p]),
